@@ -25,6 +25,13 @@ units, no data-path collective, weak scaling) - and the same JSON line carries `
 3840x2160 frames split into interleaved 16-row tiles across the ranks with the gather fused into the display kernel's
 stores (peer memory over NVLink), strong scaling; at N = 1 `config3_tiles` holds the single-GPU 4K figure the N > 1
 runs are compared with.
+
+--dump-outputs DIR   after the timed steps, what the device-resident loop (rank 0's) computed in its last step: per
+             frame the arrays run_job hands a caller, DIR/rgba8.npy [frames, pixels, 4] and DIR/depth.npy [frames,
+             pixels] (float32), so that two builds can be compared output for output.  The frames of that step are
+             copied device to device right after their display pass (inside the timed region: 8 B/px for those frames
+             only); when they exceed DUMP_BYTES, the same fixed, seeded sample of pixels (row-major index into the
+             W x H frame, row 0 at the bottom) is kept from every frame.  The inputs depend on the arguments only.
 """
 from __future__ import annotations
 
@@ -64,6 +71,7 @@ MANDELBULB_MUFU_PER_DE_TRIP = 11.0
 MANDELBULB_DE_TRIPS_PER_EVAL_PINNED = 2.44
 N_POSES = 256
 FLUSH_BYTES = 160 << 20   # > the 126 MB L2 of a B200
+DUMP_BYTES = 48 << 20     # --dump-outputs: float32 bytes written at most
 
 
 # orbit centre and radius of the synthetic camera path per scene (default: the guide scene's
@@ -271,6 +279,29 @@ def workload_config(args) -> dict:
             "steps_per_px_reference": ref_steps_per_px(args)}
 
 
+class OutputDump:
+    """--dump-outputs: device copies of the RGBA8 and depth planes of the `frames` frames of the last timed step."""
+
+    def __init__(self, torch, frames, W, H):
+        import numpy as np
+        self.rgba8 = torch.empty((frames, H * W, 4), dtype=torch.uint8, device="cuda")
+        self.depth = torch.empty((frames, H * W), dtype=torch.float32, device="cuda")
+        keep = min(H * W, DUMP_BYTES // (frames * 5 * 4))
+        # RandomState: its stream is frozen across numpy versions, so every build samples the same pixels
+        index = np.arange(H * W) if keep == H * W else np.sort(np.random.RandomState(0).permutation(H * W)[:keep])
+        self.index = torch.from_numpy(index).to("cuda")
+
+    def slot(self, k):
+        """(RGBA8, depth) device addresses for frame k of the step"""
+        return self.rgba8[k].data_ptr(), self.depth[k].data_ptr()
+
+    def write(self, directory):
+        import numpy as np
+        os.makedirs(directory, exist_ok=True)
+        np.save(os.path.join(directory, "rgba8.npy"), self.rgba8[:, self.index].float().cpu().numpy())
+        np.save(os.path.join(directory, "depth.npy"), self.depth[:, self.index].cpu().numpy())
+
+
 class Rig:
     """The contexts, programs and streams of one workload shape on this rank: (W, H, mode, tiles?)."""
 
@@ -336,8 +367,9 @@ class Rig:
         with self.torch.cuda.stream(self.streams[0]):
             self.flush_bufs[0].zero_()
 
-    def device_frame(self, frame, flush=False, nctx=None):
-        """one frame, everything resident in HBM (async): [L2 flush], uniforms, raymarch, display[, gather]"""
+    def device_frame(self, frame, flush=False, nctx=None, capture=None):
+        """one frame, everything resident in HBM (async): [L2 flush], uniforms, raymarch, display[, gather][, copy of the
+        presented RGBA8 and depth planes to the device addresses `capture`]"""
         k = frame % (nctx or self.nctx)
         ctx, prog, stream = self.ctxs[k], self.progs[k], self.streams[k]
         L, W, H, rm = self.L, self.W, self.H, self.rm
@@ -367,6 +399,10 @@ class Rig:
                 fused.complete(ctx)       # completion flag in stream order (or a one-element all-reduce): every rank has presented
             elif self.tiles and self.world > 1:
                 self._gather_tiles(ctx, stream, fb)
+        if capture:
+            for which, dst in zip((4, 3), capture):
+                st = L.rmb_fb_copy_to_device(ctx.handle, fb.handle, which, dst, fb.local_rows * W * 4)
+                assert st == 0, ctx.last_error()
         ctx.fbo.delete(W, H, s.render.frameid)
         return k
 
@@ -382,11 +418,11 @@ class Rig:
         self.dist.all_reduce(t, op=self.dist.ReduceOp.MAX)
         return float(t.item())
 
-    def measure_device(self, first_frame, n_frames, frames_per_step=1):
+    def measure_device(self, first_frame, n_frames, frames_per_step=1, dump=None):
         """n_frames enqueued back to back (the host runs ahead of the GPU); before every step (frames_per_step frames)
         an in-stream 160 MiB L2 flush, INSIDE the timed region; one start event (GPU idle,
-        recorded on every stream) to the last end event.  Returns (total ms max over ranks, launches, (evals,
-        pixel-samples, far evals))."""
+        recorded on every stream) to the last end event.  `dump` (OutputDump) receives the frames of the last step.
+        Returns (total ms max over ranks, launches, (evals, pixel-samples, far evals))."""
         torch = self.torch
         for c in self.ctxs:
             c.sync()
@@ -397,10 +433,11 @@ class Rig:
         ends = [torch.cuda.Event(enable_timing=True) for _ in self.ctxs]
         for e, st_ in zip(starts, self.streams):
             e.record(st_)
+        last_step = n_frames - max(1, frames_per_step)
         for i in range(n_frames):
             if i % max(1, frames_per_step) == 0:
                 self.flush_l2()
-            self.device_frame(first_frame + i)
+            self.device_frame(first_frame + i, capture=dump.slot(i - last_step) if dump and i >= last_step else None)
         for e, st_ in zip(ends, self.streams):
             e.record(st_)
         self.barrier()
@@ -512,12 +549,18 @@ def run_b200(args):
     for i in range(warm_frames):
         rig.device_frame(i, flush=True)
 
+    if args.dump_outputs and tiles:
+        raise SystemExit("bench.py: --dump-outputs needs whole frames on every rank (--shard poses)")
+    dump = OutputDump(torch, F, W, H) if args.dump_outputs and rank == 0 else None
+
     sampler = ClockSampler(local)
     sampler.start()
 
     # ---- timed: device-resident, K steps of F frames
     n_frames = args.steps * F
-    total_ms, gpu_launches, (evals, pxs, far_evals) = rig.measure_device(args.warmup * F, n_frames, F)
+    total_ms, gpu_launches, (evals, pxs, far_evals) = rig.measure_device(args.warmup * F, n_frames, F, dump)
+    if dump:
+        dump.write(args.dump_outputs)
     frames_all = n_frames * (1 if tiles else world)
     value = frames_all * W * H * args.spp / (total_ms * 1e-3) / 1e6     # pixel-samples per second, whole job
 
@@ -739,7 +782,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-second-flavour", action="store_true", help="do not also measure --flavour fast / far-field off beside an exact-flavour headline")
     ap.add_argument("--quick", action="store_true", help="headline + roofline only: no cpu baseline, second flavour, e2e breakdown or config 3")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the RGBA8 and depth of the last timed step's frames to DIR/*.npy (see the header)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.steps < 1):
+        ap.error("--dump-outputs needs --impl b200 and --steps >= 1")
     if args.impl == "reference":
         run_reference(args)
     else:
