@@ -109,14 +109,8 @@ rmb_status rmb_program_get(rmb_ctx* ctx, const char* scene_glsl, size_t scene_le
 int rmb_program_is_live(rmb_program* prog);
 /* generated CUDA C++ translation unit (debugging / tests); owned by the program */
 const char* rmb_program_source(rmb_program* prog);
-/* 1 if the program carries the two-rays-per-lane march kernels (packed FP32; every bundled scene without
- * position-dependent branches, swizzles or matrices in sdf()), else 0 and rmb_program_dual_log tells why
- * (compiler log of the packed attempt; the program then marches one ray per lane - same results) */
-int rmb_program_is_dual(rmb_program* prog);
-const char* rmb_program_dual_log(rmb_program* prog);
 /* registers per thread / local-memory bytes of a kernel: 0 preview megakernel, 1 full megakernel,
- * 2 preview march, 3 castRay march, 4 setup, 5 bounce (2..5: wavefront, pure scenes only), 6 / 7 the
- * two-rays-per-lane preview / castRay march; -1 if unknown */
+ * 2 preview march, 3 castRay march, 4 setup, 5 bounce (2..5: wavefront, pure scenes only); -1 if unknown */
 int rmb_program_kernel_attr(rmb_program* prog, int kernel, int* regs, int* local_bytes);
 
 /* ---- uniforms ------------------------------------------------------------------------------

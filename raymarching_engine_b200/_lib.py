@@ -20,7 +20,7 @@ UNIFORM_F, UNIFORM_I, UNIFORM_UI = 0, 1, 2
 # every symbol include/rmb.h declares; tests check that the library exports all of them
 EXPORTED_SYMBOLS = [
     "rmb_abi_version", "rmb_ctx_create", "rmb_ctx_destroy", "rmb_last_error", "rmb_ctx_stream", "rmb_sync", "rmb_ctx_set_pipeline", "rmb_ctx_launch_count", "rmb_ctx_timing", "rmb_ctx_set_gather_target", "rmb_fb_scatter_rows", "rmb_display_planes", "rmb_ipc_export", "rmb_ipc_open", "rmb_ipc_close",
-    "rmb_program_get", "rmb_program_is_live", "rmb_program_source", "rmb_program_is_dual", "rmb_program_dual_log", "rmb_program_kernel_attr", "rmb_uniform_set", "rmb_uniform_set_array",
+    "rmb_program_get", "rmb_program_is_live", "rmb_program_source", "rmb_program_kernel_attr", "rmb_uniform_set", "rmb_uniform_set_array",
     "rmb_uniform_matrix4", "rmb_fb_acquire", "rmb_fb_release", "rmb_fb_local_rows", "rmb_fb_global_row",
     "rmb_render_sample", "rmb_present", "rmb_present_device", "rmb_present_async", "rmb_present_wait", "rmb_fb_device_ptr", "rmb_fb_plane_bytes",
     "rmb_fb_read", "rmb_fb_write", "rmb_fb_copy_to_device", "rmb_counters_read", "rmb_counters_read3", "rmb_counters_read_all", "rmb_program_has_carve", "rmb_probe_carve", "rmb_probe", "rmb_compile_only", "rmb_translate_only", "rmb_host_alloc", "rmb_device_alloc", "rmb_device_free",
@@ -77,8 +77,6 @@ def _load() -> C.CDLL:
         "rmb_program_get": (i, [vp, cp, sz, i, C.POINTER(SpecUniform), i, C.POINTER(vp), cp, cp, sz]),
         "rmb_program_is_live": (i, [vp]),
         "rmb_program_source": (cp, [vp]),
-        "rmb_program_is_dual": (i, [vp]),
-        "rmb_program_dual_log": (cp, [vp]),
         "rmb_program_kernel_attr": (i, [vp, i, C.POINTER(i), C.POINTER(i)]),
         "rmb_uniform_set": (i, [vp, cp, i, i, vp]),
         "rmb_uniform_set_array": (i, [vp, cp, i, i, i, vp]),

@@ -73,19 +73,6 @@ RM_HD float g_div(float a, float b) { return __fdiv_rn(a, b); }
 RM_HD float g_sqrt(float a) { return __fsqrt_rn(a); }
 RM_HD float g_rsqrt(float a) { return __fdiv_rn(1.0f, __fsqrt_rn(a)); }
 RM_HD float g_floor(float a) { return floorf(a); }
-// floor() on the FP32 + integer pipes, bit-identical to floorf for EVERY input: round-down add of
-// 1.5*2^23 (its ulp is 1, so the sum is floor(a) + M exactly for |a| <= 2^22), subtract, restore the
-// sign of a zero result (floor(-0) = -0, floor(0.3) = +0, floor(-0.3) = -1 is already negative), and
-// leave |a| > 2^22 / inf / NaN to FRND behind a branch that is practically never taken.  FRND issues on
-// the 16-lane XU pipe, which the exact flavour's march loop saturates together with the issue slots;
-// the vector mod() below moves RM_FLOOR_FP_COMPONENTS of its three floors here to balance the pipes.
-RM_HD float g_floor_fp(float a) {
-    const float M = 12582912.0f;
-    float r = __fadd_rn(__fadd_rd(a, M), -M);
-    r = __uint_as_float(__float_as_uint(r) | (__float_as_uint(a) & 0x80000000u));
-    if (!(fabsf(a) <= 4194304.0f)) r = floorf(a);
-    return r;
-}
 RM_HD float g_fma(float a, float b, float c) { return __fmaf_rn(a, b, c); }
 #if defined(RM_FLAVOUR_FAST) && RM_FLAVOUR_FAST
 // inside a fast-flavour program (--prec-div=false) the exact namespace must not depend on flags
@@ -106,7 +93,7 @@ RM_HD float g_fma(float a, float b, float c) { return __builtin_fmaf(a, b, c); }
 RM_HD float g_rcp(float a) { return 1.0f / a; }
 #endif
 
-#if RM_DEVICE_CODE && defined(RM_USE_F32X2) && RM_USE_F32X2
+#if RM_DEVICE_CODE
 // Blackwell packed FP32 (FFMA2 / FADD2 / FMUL2: two IEEE round-to-nearest operations per lane per issue
 // slot, bit-identical to the scalar instructions).  The march loops are issue-bound, so the x and y
 // components of the hot vector operations travel as one f32x2 value; z stays scalar.
@@ -511,20 +498,7 @@ GLSL_MAP1(exp) GLSL_MAP1(log) GLSL_MAP1(exp2) GLSL_MAP1(log2) GLSL_MAP1(sqrt) GL
 GLSL_MAP1(abs) GLSL_MAP1(sign) GLSL_MAP1(floor) GLSL_MAP1(trunc) GLSL_MAP1(round) GLSL_MAP1(roundEven)
 GLSL_MAP1(ceil) GLSL_MAP1(fract)
 GLSL_MAP2(atan) GLSL_MAP2(pow) GLSL_MAP2(mod) GLSL_MAP2(min) GLSL_MAP2(max)
-GLSL_MAP2S(min) GLSL_MAP2S(max)
-#if !GLSL_FAST && RM_DEVICE_CODE && defined(RM_FLOOR_FP_COMPONENTS) && !(defined(RM_PIN_ALT) && RM_PIN_ALT)
-// exact device policy: same value as mod(float, float), with the floor of the first
-// RM_FLOOR_FP_COMPONENTS components evaluated off the XU pipe (g_floor_fp)
-RM_HD float mod_fp(float x, float y) { return g_fma(-y, g_floor_fp(g_mul(x, g_rcp(y))), x); }
-RM_HD vec2 mod(const vec2& a, float b) { return vec2(RM_FLOOR_FP_COMPONENTS > 0 ? mod_fp(a.x, b) : mod(a.x, b), RM_FLOOR_FP_COMPONENTS > 1 ? mod_fp(a.y, b) : mod(a.y, b)); }
-RM_HD vec3 mod(const vec3& a, float b) {
-    return vec3(RM_FLOOR_FP_COMPONENTS > 0 ? mod_fp(a.x, b) : mod(a.x, b), RM_FLOOR_FP_COMPONENTS > 1 ? mod_fp(a.y, b) : mod(a.y, b),
-                RM_FLOOR_FP_COMPONENTS > 2 ? mod_fp(a.z, b) : mod(a.z, b));
-}
-RM_HD vec4 mod(const vec4& a, float b) { return vec4(mod(a.x, b), mod(a.y, b), mod(a.z, b), mod(a.w, b)); }
-#else
-GLSL_MAP2S(mod)
-#endif
+GLSL_MAP2S(min) GLSL_MAP2S(max) GLSL_MAP2S(mod)
 #undef GLSL_MAP1
 #undef GLSL_MAP2
 #undef GLSL_MAP2S
@@ -537,7 +511,7 @@ RM_HD float rm_c(const vec4& a, int i) { return a[i]; }
 template <class H1, class S, class H2> RM_HD vec2 rm_rep(const vec2& x, const H1& h1, const S& s, const H2& h2) {
     return vec2(rm_rep1(x.x, rm_c(h1, 0), rm_c(s, 0), rm_c(h2, 0)), rm_rep1(x.y, rm_c(h1, 1), rm_c(s, 1), rm_c(h2, 1)));
 }
-#if !GLSL_FAST && GLSL_F32X2 && !(defined(RM_PIN_ALT) && RM_PIN_ALT) && !(defined(RM_FLOOR_FP_COMPONENTS) && RM_FLOOR_FP_COMPONENTS > 0)
+#if !GLSL_FAST && GLSL_F32X2 && !(defined(RM_PIN_ALT) && RM_PIN_ALT)
 // exact policy, packed: the same operations as rm_rep1 on every component - add, multiply by the
 // correctly rounded reciprocal, floor, fused multiply-add, subtract - with x and y sharing FADD2 /
 // FMUL2 / FFMA2 instructions (IEEE round-to-nearest per element, so the bits are those of rm_rep1)
@@ -557,15 +531,7 @@ template <class H1, class S, class H2> RM_HD vec3 rm_rep(const vec3& x, const H1
     (void)rz;
     return out;
 }
-#elif !GLSL_FAST && RM_DEVICE_CODE && defined(RM_FLOOR_FP_COMPONENTS) && !(defined(RM_PIN_ALT) && RM_PIN_ALT)
-RM_HD float rm_rep1_fp(float x, float h1, float s, float h2) { return g_sub(mod_fp(g_add(x, h1), s), h2); }
-template <class H1, class S, class H2> RM_HD vec3 rm_rep(const vec3& x, const H1& h1, const S& s, const H2& h2) {
-    return vec3(RM_FLOOR_FP_COMPONENTS > 0 ? rm_rep1_fp(x.x, rm_c(h1, 0), rm_c(s, 0), rm_c(h2, 0)) : rm_rep1(x.x, rm_c(h1, 0), rm_c(s, 0), rm_c(h2, 0)),
-                RM_FLOOR_FP_COMPONENTS > 1 ? rm_rep1_fp(x.y, rm_c(h1, 1), rm_c(s, 1), rm_c(h2, 1)) : rm_rep1(x.y, rm_c(h1, 1), rm_c(s, 1), rm_c(h2, 1)),
-                RM_FLOOR_FP_COMPONENTS > 2 ? rm_rep1_fp(x.z, rm_c(h1, 2), rm_c(s, 2), rm_c(h2, 2)) : rm_rep1(x.z, rm_c(h1, 2), rm_c(s, 2), rm_c(h2, 2)));
-}
-#else
-#if GLSL_FAST && GLSL_F32X2
+#elif GLSL_FAST && GLSL_F32X2
 // packed (x, y) + scalar z version of the centred remainder
 template <class H1, class S, class H2> RM_HD vec3 rm_rep(const vec3& x, const H1& h1, const S& s, const H2& h2) {
     const float s0 = rm_c(s, 0), a0 = rm_c(h1, 0), b0 = rm_c(h2, 0);
@@ -589,7 +555,6 @@ template <class H1, class S, class H2> RM_HD vec3 rm_rep(const vec3& x, const H1
     return vec3(rm_rep1(x.x, rm_c(h1, 0), rm_c(s, 0), rm_c(h2, 0)), rm_rep1(x.y, rm_c(h1, 1), rm_c(s, 1), rm_c(h2, 1)),
                 rm_rep1(x.z, rm_c(h1, 2), rm_c(s, 2), rm_c(h2, 2)));
 }
-#endif
 #endif
 template <class H1, class S, class H2> RM_HD vec4 rm_rep(const vec4& x, const H1& h1, const S& s, const H2& h2) {
     return vec4(rm_rep1(x.x, rm_c(h1, 0), rm_c(s, 0), rm_c(h2, 0)), rm_rep1(x.y, rm_c(h1, 1), rm_c(s, 1), rm_c(h2, 1)),
@@ -648,12 +613,6 @@ RM_HD float rm_rep1_nf(float x, float h1, float s, float h2) {
     const float a = g_add(x, h1);
     return g_sub(g_fma(-s, g_floor_nf(g_mul(a, g_rcp(s)), h2), a), h2);
 }
-#if !GLSL_F32X2
-template <class H1, class S, class H2> RM_HD vec3 rm_rep_nf(const vec3& x, const H1& h1, const S& s, const H2& h2) {
-    return vec3(rm_rep1_nf(x.x, rm_c(h1, 0), rm_c(s, 0), rm_c(h2, 0)), rm_rep1_nf(x.y, rm_c(h1, 1), rm_c(s, 1), rm_c(h2, 1)),
-                rm_rep1_nf(x.z, rm_c(h1, 2), rm_c(s, 2), rm_c(h2, 2)));
-}
-#else
 // the packed rm_rep (above) with that floor: FADD2 / FMUL2 / FADD2.RM / FADD2 / FFMA2 / FADD2 for x and y
 template <class H1, class S, class H2> RM_HD vec3 rm_rep_nf(const vec3& x, const H1& h1, const S& s, const H2& h2) {
     const float M = 12582912.0f;
@@ -670,7 +629,6 @@ template <class H1, class S, class H2> RM_HD vec3 rm_rep_nf(const vec3& x, const
     out.z = rm_rep1_nf(x.z, rm_c(h1, 2), sz, rm_c(h2, 2));
     return out;
 }
-#endif
 #endif
 
 RM_HD vec2 clamp(const vec2& v, float lo, float hi) { return vec2(clamp(v.x, lo, hi), clamp(v.y, lo, hi)); }

@@ -1064,100 +1064,6 @@ LowerResult lower_scene(const std::string& glsl, const std::set<std::string>& co
         }
     }
 
-    // ---- pass 3: "varying" lowering for the packed (two rays per lane) march kernels -------------
-    // Works on a copy of the token texts; see LowerResult::body_packed and device_src/glsl_pk.h.
-    std::vector<std::string> packed_text(n);
-    for (size_t k = 0; k < n; k++) packed_text[k] = T[k].text;
-    for (size_t k : carve.rep_sites) packed_text[k] = T[k].text == "rm_rep_b" ? "rm_rep" : "rm_rep0";
-    {
-        auto live = [&](size_t k) { return k < n && !T[k].drop && T[k].kind != kPP; };
-        auto next_live = [&](size_t k) { k++; while (k < n && !live(k)) k++; return k; };
-        auto prev_live = [&](size_t k) -> size_t { while (k > 0) { k--; if (live(k)) return k; } return n; };
-        static const std::set<std::string> fvec = {"float", "vec2", "vec3", "vec4"};
-        auto base_type = [](std::string t) { if (!t.empty() && t.back() == '&') t.pop_back(); return t; };
-        char bt; int bc;
-        int depth = 0;
-        for (size_t k = 0; k < n; k++) {
-            if (!live(k)) continue;
-            const std::string& w = T[k].text;
-            if (T[k].kind == kPunct) {
-                if (w == "{") depth++;
-                else if (w == "}") depth--;
-                continue;
-            }
-            if (T[k].kind != kIdent) continue;
-            if (depth == 0) {
-                // function definition:  [const] TYPE NAME ( params ) {
-                size_t ty = k;
-                if (w == "const") ty = next_live(k);
-                if (ty >= n || T[ty].kind != kIdent) continue;
-                const std::string rtype = T[ty].text;
-                if (!(uniform_type_info(rtype, &bt, &bc) || rtype == "void")) continue;
-                size_t name = next_live(ty), open = name < n ? next_live(name) : n;
-                if (name >= n || open >= n || T[name].kind != kIdent || T[open].text != "(") continue;
-                size_t close = open; int d = 0;
-                for (size_t q = open; q < n; q++) {
-                    if (!live(q)) continue;
-                    if (T[q].text == "(") d++;
-                    if (T[q].text == ")") { d--; if (d == 0) { close = q; break; } }
-                }
-                size_t after = next_live(close);
-                if (close == open || after >= n || T[after].text != "{") { k = close; continue; }   // prototype: left alone
-                // parameters: [const] TYPE[&] NAME, separated by commas
-                std::string tmpl;
-                int np = 0;
-                bool ok = true;
-                size_t q = next_live(open);
-                while (q < close && ok) {
-                    if (T[q].text == "const") q = next_live(q);
-                    if (q >= close || T[q].kind != kIdent || !(uniform_type_info(base_type(T[q].text), &bt, &bc))) { ok = (q >= close) || T[q].text == "void"; break; }
-                    const bool ref = T[q].text.back() == '&';
-                    size_t pn = next_live(q);
-                    if (pn >= close || T[pn].kind != kIdent) { ok = false; break; }
-                    size_t sep = next_live(pn);
-                    if (sep < close && T[sep].text != ",") { ok = false; break; }     // arrays etc.: not handled
-                    if (fvec.count(base_type(T[q].text))) {
-                        packed_text[q] = "RM_P" + std::to_string(np) + (ref ? "&" : "");
-                        tmpl += std::string(np ? ", " : "") + "class RM_P" + std::to_string(np);
-                        np++;
-                    }
-                    q = sep < close ? next_live(sep) : close;
-                }
-                if (!ok) { k = close; continue; }
-                if (rtype != "void" && fvec.count(rtype)) packed_text[ty] = "auto";
-                if (np) packed_text[k] = "template <" + tmpl + "> " + packed_text[k];
-                k = close;
-                continue;
-            }
-            // inside a function body
-            if (fvec.count(w)) {
-                size_t nx = next_live(k);
-                if (nx < n && T[nx].text == "(") {                 // constructor / conversion call
-                    packed_text[k] = "rm_" + w;
-                    continue;
-                }
-                if (nx >= n || T[nx].kind != kIdent) continue;
-                size_t pv = prev_live(k);
-                if (pv != n && T[pv].text == "const") pv = prev_live(pv);
-                if (pv != n && T[pv].text == "(") {
-                    size_t pp = prev_live(pv);
-                    // (pass 1 may have prefixed the keyword with an unroll pragma)
-                    if (pp != n && T[pp].text.size() >= 3 && T[pp].text.compare(T[pp].text.size() - 3, 3, "for") == 0) continue;  // loop counter: stays a plain float
-                }
-                size_t aft = next_live(nx);
-                if (aft >= n) continue;
-                if (T[aft].text == ";") { packed_text[k] = "RM_ACC_" + w; continue; }
-                if (T[aft].text != "=") continue;
-                // initialiser: a lone numeric literal (an accumulator that varying values will be assigned to)?
-                size_t v = next_live(aft);
-                if (v < n && (T[v].text == "-" || T[v].text == "+")) v = next_live(v);
-                size_t endv = v < n ? next_live(v) : n;
-                if (v < n && T[v].kind == kNumber && endv < n && T[endv].text == ";") packed_text[k] = "RM_ACC_" + w;
-                else packed_text[k] = "auto";
-            }
-        }
-    }
-
     // ---- emit -------------------------------------------------------------------------------
     std::string out;
     out.reserve(glsl.size() + 256);
@@ -1170,19 +1076,6 @@ LowerResult lower_scene(const std::string& glsl, const std::set<std::string>& co
     }
     out += trailing;
     R.body = out;
-    {
-        std::string pk;
-        pk.reserve(out.size() + 512);
-        for (size_t k = 0; k < n; k++) {
-            const Token& t = T[k];
-            pk += t.ws;
-            if (t.drop) continue;
-            if (!pk.empty() && is_ident_char(pk.back()) && !packed_text[k].empty() && is_ident_char(packed_text[k][0]) && t.ws.empty()) pk += ' ';
-            pk += packed_text[k];
-        }
-        pk += trailing;
-        R.body_packed = pk;
-    }
 
     if (carve.ok) {
         // helper functions (members of the fragment struct, after the scene): token texts as they stand

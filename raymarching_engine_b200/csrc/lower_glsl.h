@@ -21,10 +21,6 @@ struct LowerResult {
     bool ok = false;
     std::string error;                  // GL-style message when !ok
     std::string body;                   // lowered scene text, same line structure as the input
-    std::string body_packed;            // the same scene lowered for the two-rays-per-lane march kernels:
-                                        // functions are templates over their parameter types and initialised
-                                        // locals are `auto`, so values derived from the ray position become the
-                                        // packed types of glsl_pk.h while uniform-only expressions stay float
     std::vector<UniformDecl> uniforms;  // scene-declared uniforms, removed from `body`
     std::set<std::string> functions;    // functions DEFINED at global scope
     std::set<std::string> macros;       // names the scene #defines: the translation unit #undefs them after the scene text,

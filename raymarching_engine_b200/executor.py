@@ -41,16 +41,9 @@ class Program:
     def source(self) -> str:
         return L.rmb_program_source(self.handle).decode()
 
-    def is_dual(self) -> bool:
-        """True when the program marches two rays per lane with packed FP32 (glsl_pk.h)"""
-        return bool(L.rmb_program_is_dual(self.handle))
-
     def has_carve(self) -> bool:
         """True when the march kernels take the far-field shortcut of a carved scene (include/rmb.h)"""
         return bool(L.rmb_program_has_carve(self.handle))
-
-    def dual_log(self) -> str:
-        return (L.rmb_program_dual_log(self.handle) or b"").decode()
 
     def kernel_attr(self, kernel: int):
         r, l = C.c_int(-1), C.c_int(-1)

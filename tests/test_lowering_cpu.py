@@ -1,6 +1,7 @@
 """GLSL -> CUDA lowering and NVRTC compilation for sm_100a, exercised without a GPU
 (NVRTC is a compiler; rmb_compile_only never touches a device)."""
 import ctypes as C
+import re
 
 import pytest
 
@@ -115,7 +116,8 @@ def test_compile_errors_are_values_with_gl_style_lines():
 
 def test_translate_only_reports_scene_level_errors_without_compiling():
     """rmb_translate_only: the lowering alone (milliseconds) gives the scene-level diagnostics and the translation unit;
-    errors only the C++ compiler can see (an undeclared identifier) need rmb_compile_only."""
+    errors only the C++ compiler can see (an undeclared identifier) need rmb_compile_only.  The march has one
+    implementation with fixed tunables: the translation unit carries no switch for them."""
     def translate(src):
         log = C.create_string_buffer(1 << 16)
         out = C.create_string_buffer(2 << 20)
@@ -124,6 +126,10 @@ def test_translate_only_reports_scene_level_errors_without_compiling():
         return st, log.value.decode(), out.value.decode()
     st, log, tu = translate(scene_source("guide"))
     assert st == _lib.RMB_OK and "rm_wf_march_preview_kernel" in tu and "__constant__ float fractalIterations;" in tu
+    for name in ("RM_DUAL", "scene_packed.glsl", "RM_FLOOR_FP_COMPONENTS", "RM_WF_CHUNK", "RM_REFILL_MIN", "RM_MARCH_MIN_BLOCKS",
+                 "RM_BOUNCE_MIN_BLOCKS", "RM_USE_F32X2"):
+        assert name not in tu, name
+    assert set(re.findall(r"\bRMB_\w+", tu)) <= {"RMB_PROFILE"}    # the kernel text names only the profiling switch
     st, log, _ = translate("vec3 sceneEmission(vec3 p) { return vec3(0.0); }\n")
     assert st == _lib.RMB_ERR_FRAGMENT and "'sdf'" in log
     st, log, _ = translate("uniform sampler2D tex;\nfloat sdf(vec3 p) { return 1.0; }")
@@ -151,37 +157,6 @@ float sdf(vec3 p) {
     st, log, _, tu = compile_only(src)
     assert st == _lib.RMB_OK, log
     assert "__constant__ float weights[4];" in tu and "__constant__ ivec3 cell;" in tu and "__constant__ mat3 basis;" in tu
-
-
-def test_varying_lowering_for_the_two_rays_per_lane_kernels(monkeypatch):
-    """RMB_DUAL=1: the scene is lowered a second time with functions as templates over their parameter
-    types and initialised locals as `auto` (uniform-only expressions stay float and fold; everything
-    derived from the position becomes the packed types of glsl_pk.h), and the dual march kernels compile
-    for sm_100a.  Scenes the lowering cannot express fall back to the one-ray program."""
-    monkeypatch.setenv("RMB_DUAL", "1")
-    src = scene_source("guide")
-    st, log, nbytes, tu = compile_only(src, _lib.FLAVOUR_EXACT, rm.default_custom_settings(src))
-    assert st == _lib.RMB_OK, log
-    assert "#define RM_DUAL 1" in tu
-    packed = tu[tu.index('#line 1 "scene_packed.glsl"'):]
-    assert "template <class RM_P0> auto sdf(RM_P0 position)" in packed
-    assert "RM_ACC_float minDist = 9999.9f;" in packed                      # literal-initialised accumulator -> packed
-    assert "for (float i = -1.0f; i < fractalIterations; i++)" in packed    # loop counters stay uniform
-    assert "auto sf = pow(gridScaleFactor, i);" in packed                   # uniform-only: stays float, folds
-    assert "rm_vec3(0.5f * sf)" in packed and "auto d = abs(rm_rep(position" in packed
-    # fast flavour too
-    st, log, _, tu = compile_only(src, _lib.FLAVOUR_FAST, rm.default_custom_settings(src))
-    assert st == _lib.RMB_OK and "#define RM_DUAL 1" in tu, log
-    # swizzles / matrices / position-dependent branches: packed attempt fails, one-ray program is built
-    for name in ("tree", "mandelbulb"):
-        s2 = scene_source(name)
-        st, log, nbytes, tu = compile_only(s2, _lib.FLAVOUR_EXACT, rm.default_custom_settings(s2))
-        assert st == _lib.RMB_OK and nbytes > 10000, log
-        assert "#define RM_DUAL 0" in tu
-    # strict mode reports why
-    monkeypatch.setenv("RMB_DUAL_STRICT", "1")
-    st, log, _, _ = compile_only(scene_source("tree"), _lib.FLAVOUR_EXACT, rm.default_custom_settings(scene_source("tree")))
-    assert st != _lib.RMB_OK and "pvec3" in log
 
 
 def test_preprocessor_directives_are_sandboxed():

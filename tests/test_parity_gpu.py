@@ -572,43 +572,6 @@ def test_render_frames_two_contexts_equals_run_job(ctx):
         other.close()
 
 
-@pytest.mark.parametrize("name,dual_expected", [("guide", True), ("menger-sponge", True), ("tree", False)])
-def test_two_rays_per_lane_march_is_bit_identical(ctx, name, dual_expected, monkeypatch):
-    """RMB_DUAL=1 builds the march kernels that carry two rays per lane and evaluate the scene's SDF with
-    packed FP32 instructions for both (glsl_pk.h + the "varying" lowering).  Same bits as the default
-    one-ray kernels; scenes the varying lowering cannot express (tree: swizzles, matrices) silently
-    keep the one-ray kernels."""
-    src = scene_source(name)
-    custom = rm.default_custom_settings(src)
-    outs = []
-    monkeypatch.setenv("RMB_CARVE", "0")                # the far-field pipeline of carved scenes uses the one-ray kernels
-    for dual in ("0", "1"):
-        monkeypatch.setenv("RMB_DUAL", dual)
-        c = rm.load_render_job_context(device=0)      # programs are cached per context: fresh context per setting
-        try:
-            prog = c.program_cache.get_program(src, None, custom)
-            assert isinstance(prog, rm.Program), prog
-            assert prog.is_dual() == (dual == "1" and dual_expected), prog.dual_log()[:400]
-            frames = []
-            for mode in ("preview", "full"):
-                s = rm.default_schema(src, custom, width=200, height=112, renderMode=mode, frameid=9900 + len(outs) * 10 + len(frames))
-                if mode == "full":
-                    s.lights = [rm.default_light()]
-                rm.reset_halton()
-                fb = c.fbo.create(200, 112, s.render.frameid)
-                got = rm.run_job(s, c)
-                assert got["success"], got["why"]
-                frames.append((fb.read("color"), fb.read("depth"), got["rgba8"].copy(), c.counters(reset=True)))
-            outs.append(frames)
-        finally:
-            c.close()
-    for a, b in zip(outs[0], outs[1]):
-        np.testing.assert_array_equal(_canon(a[0]), _canon(b[0]))
-        np.testing.assert_array_equal(_canon(a[1]), _canon(b[1]))
-        np.testing.assert_array_equal(a[2], b[2])
-        assert a[3] == b[3]                             # same number of SDF evaluations and pixel-samples
-
-
 def _carve_points(rng, centre, radius):
     c = np.asarray(centre, np.float32)
     near = c + rng.uniform(-1.3, 1.3, (60000, 3)).astype(np.float32) * np.float32(radius)

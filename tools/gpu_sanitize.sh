@@ -1,7 +1,7 @@
 #!/bin/bash
 # usage: bash tools/gpu_sanitize.sh [tag] : compute-sanitizer memcheck + racecheck over small preview + full renders through the
-# public API, once per build / launch switch that changes which kernels or buffers are in play: defaults, RMB_WF_ORDER=1 (tile
-# order list), RMB_DUAL=1 (two rays per lane), RMB_CARVE=0 (no far-field pipeline), a multi-pass march plan with step budgets, a
+# public API, once per build / launch switch that changes which kernels or buffers are in play: defaults, RMB_CARVE=0 (no
+# far-field pipeline), a multi-pass march plan with step budgets, a
 # device group of two members on this GPU (tile contexts, fused gather store, row scatter), and frame sizes that make the ray
 # planes / record lists grow between draws.  Logs -> gpurun_out/sanitizer_<tag>_<case>_<tool>.log
 TAG=${1:-r2}
@@ -37,8 +37,6 @@ run() {   # name, env...
   done
 }
 run defaults SAN_X=0
-run wf_order RMB_WF_ORDER=1
-run dual RMB_DUAL=1
 run no_carve RMB_CARVE=0
 run plan_budget RMB_MARCH_PLAN=24:256:2:8,0:128:1:0
 run group2 SAN_GROUP=1

@@ -2,7 +2,7 @@
 """One-process sweep of RMB_MARCH_PLAN (rmb_api.cpp "march stage": budget:threads:ctas_per_sm:pause per pass) on the
 default bench workload: frames of the orbit path, one context, L2 flushed per frame, march-kernel time from the
 library's CUDA-event timer and frame time from events around the whole sequence.  The plan is read at every draw, so
-no recompilation is needed between rows (RMB_REFILL_MIN is compile-time: pass --refill to rebuild per value).
+no recompilation is needed between rows.
 
   python tools/sweep_plan.py [--width 1920 --height 1080] [--mode preview] [--steps 12] plan [plan ...]
 """
