@@ -811,6 +811,15 @@ int orc_materials(const char* scene, const float* custom, int ncustom, float x, 
     return -1;
 }
 
+// orc_materials at n points: xyz = n * 3 floats, out = n * 17 floats
+int orc_materials_n(const char* scene, const float* custom, int ncustom, const float* xyz, int n, float* out) {
+    for (int i = 0; i < n; i++) {
+        const int st = orc_materials(scene, custom, ncustom, xyz[3 * (size_t)i], xyz[3 * (size_t)i + 1], xyz[3 * (size_t)i + 2], out + 17 * (size_t)i);
+        if (st != 0) return st;
+    }
+    return 0;
+}
+
 unsigned long long orc_sdf_evals_reset() { return g_sdf_evals.exchange(0); }
 
 float orc_sdbox(float px, float py, float pz, float bx, float by, float bz) { return sdBox(vec3(px, py, pz), vec3(bx, by, bz)); }

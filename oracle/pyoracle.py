@@ -61,6 +61,7 @@ def lib() -> C.CDLL:
         L.orc_de_iterations_reset.restype = C.c_ulonglong
         L.orc_scene_name.restype = C.c_char_p
         L.orc_materials.argtypes = [C.c_char_p, C.c_void_p, C.c_int, C.c_float, C.c_float, C.c_float, C.c_void_p]
+        L.orc_materials_n.argtypes = [C.c_char_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p]
         L.orc_render_sample.argtypes = [C.c_char_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
                                         C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
         L.orc_display.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_void_p, C.c_int]
@@ -175,6 +176,18 @@ def executed_work(scene: str, schema, rand_noise=(0.5, 1.0 / 3.0)):
     if st != 0:
         raise RuntimeError(f"oracle exit_steps({scene}) failed: {st}")
     return int(out.sum()), int(L.orc_de_iterations_reset())
+
+
+def materials(scene: str, custom, points) -> np.ndarray:
+    """orc_materials at every point: n x 17 (the layout of the device probe kernel rmb_probe)"""
+    pts = np.ascontiguousarray(points, dtype=np.float32).reshape(-1, 3)
+    out = np.zeros((len(pts), 17), np.float32)
+    cu = flatten_custom(scene, custom)
+    st = lib().orc_materials_n(scene.encode(), cu.ctypes.data_as(C.c_void_p) if cu.size else None, int(cu.size),
+                               pts.ctypes.data_as(C.c_void_p), len(pts), out.ctypes.data_as(C.c_void_p))
+    if st != 0:
+        raise RuntimeError(f"oracle materials({scene}) failed: {st}")
+    return out
 
 
 def halton_seq(base: int, n: int) -> list:

@@ -5,7 +5,8 @@ on the LOWERED TEXT itself: the scene functions and the two helpers the lowering
 translation unit rmb_compile_only returns, compiled with g++ against the shared deterministic math
 (glsl_rt.h, exact policy, the oracle's flags) and evaluated at a few hundred thousand positions, including
 the non-finite ones escaping rays reach.  The GPU side of the same claim is tests/test_parity_gpu.py
-(test_carve_*: probe kernel, far-field on/off frames, oracle parity of every scene with the shortcut on).
+(test_carve_*: probe kernel, far-field on/off frames, oracle parity of every scene with the shortcut on) and, at the
+settings-tab value sets of tests/slider_cases.py that both files also run here, tests/test_slider_values_gpu.py.
 """
 import ctypes as C
 import os
@@ -18,6 +19,7 @@ import pytest
 
 import raymarching_engine_b200 as rm
 from raymarching_engine_b200 import _lib
+import slider_cases
 from conftest import scene_source
 
 L = _lib.lib
@@ -245,8 +247,9 @@ int main(int argc, char** argv) {
 
 
 def _cxx_value(v):
+    # bit-pattern literals, as rmb_api.cpp float_literal bakes them: NaN and +-inf uniforms compile too
     a = np.atleast_1d(np.asarray(v, dtype=np.float32))
-    lit = ["%sf" % np.format_float_scientific(x, unique=True) for x in a]
+    lit = ["__builtin_bit_cast(float, 0x%08xu)" % b for b in a.view(np.uint32)]
     return lit[0] if len(lit) == 1 else "vec%d(%s)" % (len(lit), ", ".join(lit))
 
 
@@ -288,9 +291,30 @@ def _run(exe, pts):
     return np.frombuffer(r.stdout, np.float32).reshape(-1, 3)
 
 
-@pytest.mark.parametrize("case", ["guide-defaults", "guide-varied", "inline-default", "menger-sponge", "boxes-varied"])
+SLIDER_CASES = ["%s/%s" % sc for sc in slider_cases.all_cases(slider_cases.CARVED)]
+
+
+def _slider_case(case):
+    """(source, plain uniform values, scene, case name) of a tests/slider_cases.py entry `scene/case`"""
+    scene, name = case.split("/")
+    src = scene_source(scene)
+    return src, slider_cases.plain(slider_cases.custom(rm, src, scene, name)), scene, name
+
+
+@pytest.mark.parametrize("case", ["guide-defaults", "guide-varied", "inline-default", "menger-sponge", "boxes-varied"] + SLIDER_CASES)
 def test_far_field_value_is_the_outer_shape_bit_for_bit(tmp_path, case):
     rng = np.random.default_rng(20261017)
+    if "/" in case:         # the settings-tab value sets: U as tabulated, the claim everywhere, no non-vacuity bar
+        src, values, scene, name = _slider_case(case)
+        exe = _build_harness(tmp_path, src, values)
+        out = _run(exe, _points(rng, *slider_cases.region(scene, values)))
+        sdf, A, U = out[:, 0], out[:, 1], out[:, 2]
+        assert np.all(U.view(np.uint32) == U[0].view(np.uint32))
+        assert U[0].view(np.uint32) == slider_cases.expected_U(scene, name).view(np.uint32), U[0]
+        with np.errstate(invalid="ignore"):
+            far = A > U[0]
+        np.testing.assert_array_equal(sdf[far].view(np.uint32), A[far].view(np.uint32))
+        return
     if case == "menger-sponge":
         src = scene_source("menger-sponge")
         values = {k: (v.data[0] if v.count == 1 else tuple(v.data)) for k, v in rm.default_custom_settings(src).items()}
@@ -426,10 +450,14 @@ def _build_nf_harness(tmp_path, src, values):
     return exe
 
 
-@pytest.mark.parametrize("case", ["guide-defaults", "guide-varied", "guide-tiny-cells", "inline-default"])
+@pytest.mark.parametrize("case", ["guide-defaults", "guide-varied", "guide-tiny-cells", "inline-default"] + SLIDER_CASES)
 def test_guard_free_floor_is_floorf_inside_the_proven_range(tmp_path, case):
     rng = np.random.default_rng(7)
-    if case == "inline-default":
+    scene = None
+    if "/" in case:
+        src, values, scene, _name = _slider_case(case)
+        centre, radius = slider_cases.region(scene, values)
+    elif case == "inline-default":
         src, values, centre, radius = scene_source("inline-default"), {}, (0, 0, 0), 5.0
     else:
         src = scene_source("guide")
@@ -442,8 +470,11 @@ def test_guard_free_floor_is_floorf_inside_the_proven_range(tmp_path, case):
     exe = _build_nf_harness(tmp_path, src, values)
     pts = _points(rng, centre, radius)
     # plus positions on and around cell boundaries, negative zero and tiny negatives (the floor's own edge cases)
-    cells = (rng.integers(-40, 40, (20000, 3)) * np.float32(1.0 / 3.0) ** rng.integers(0, 8, (20000, 1))).astype(np.float32)
-    cells = np.concatenate([cells, np.nextafter(cells, np.float32(-np.inf)), np.nextafter(cells, np.float32(np.inf)), -cells])
+    if scene is None:
+        cells = (rng.integers(-40, 40, (20000, 3)) * np.float32(1.0 / 3.0) ** rng.integers(0, 8, (20000, 1))).astype(np.float32)
+        cells = np.concatenate([cells, np.nextafter(cells, np.float32(-np.inf)), np.nextafter(cells, np.float32(np.inf)), -cells])
+    else:                   # the case's own cell sizes, and the band where the proven range ends
+        cells = np.concatenate([slider_cases.cell_points(rng, scene, values), slider_cases.band_points(rng)])
     edge = np.array([[-0.0, -0.0, -0.0], [-1e-45, 1e-45, -1e-40], [-0.5, -0.5, -0.5], [-1.5, -0.16666667, -0.055555556]], np.float32)
     pts = np.ascontiguousarray(np.concatenate([pts, cells, edge]).astype(np.float32))
     blob = np.uint32(len(pts)).tobytes() + pts.tobytes()
@@ -451,13 +482,16 @@ def test_guard_free_floor_is_floorf_inside_the_proven_range(tmp_path, case):
     raw = np.frombuffer(r.stdout, np.float32)
     out, max_q = raw[:-1].reshape(-1, 3), raw[-1]
     plim = out[0, 2]
-    assert np.isfinite(plim) and plim > 0
     with np.errstate(invalid="ignore"):
         inside = np.nanmax(np.abs(pts), axis=1) <= plim
     inside &= ~np.isnan(pts).all(axis=1)
-    if case != "guide-tiny-cells":
-        assert inside.sum() > 200000
-    assert inside.sum() > 1000 and (~inside).sum() > 1000
+    if scene is not None:   # a NaN or zero cell gives -1 (never fast), a loop that does not run 3e38
+        assert plim == -1.0 or (np.isfinite(plim) and plim > 0), plim
+    else:
+        assert np.isfinite(plim) and plim > 0
+        if case != "guide-tiny-cells":
+            assert inside.sum() > 200000
+        assert inside.sum() > 1000 and (~inside).sum() > 1000
     np.testing.assert_array_equal(out[inside, 0].view(np.uint32), out[inside, 1].view(np.uint32))
     assert max_q <= 4194304.0
     # not vacuous: where the limit is smaller than the carved sphere the guard-free floor really goes wrong outside it
