@@ -12,7 +12,7 @@
  * Images are row-major with row 0 at the BOTTOM (OpenGL convention), RGBA interleaved.
  * One context drives one GPU (one process per GPU; multi-GPU jobs shard rows, see rank/n_ranks).
  * All calls are asynchronous on the context's stream except rmb_present, rmb_fb_read,
- * rmb_counters_read, rmb_sync and rmb_ctx_destroy.
+ * rmb_counters_read_all, rmb_sync and rmb_ctx_destroy.
  */
 #ifndef RMB_H_
 #define RMB_H_
@@ -227,13 +227,11 @@ rmb_status rmb_fb_write(rmb_ctx* ctx, rmb_fb* fb, int which, const void* host, s
 /* asynchronous device-to-device copy of a plane on the context's stream (multi-GPU tile gather:
  * the caller hands the destination to NCCL in the same stream order) */
 rmb_status rmb_fb_copy_to_device(rmb_ctx* ctx, rmb_fb* fb, int which, void* dst_device, size_t bytes);
-/* out[0] = SDF evaluations executed, out[1] = pixel-samples rendered, since the last reset */
-rmb_status rmb_counters_read(rmb_ctx* ctx, uint64_t out[2], int reset);
-/* the same plus out[2] = how many of out[0] took the far-field shortcut of a carved scene (below) */
-rmb_status rmb_counters_read3(rmb_ctx* ctx, uint64_t out[3], int reset);
-/* all 16 counter slots: [0..2] as above; [3..11] are filled only by programs built with RMB_PROFILE=1 in the
- * environment (a measurement aid of the march kernel, see tools/march_timeline.py): warp-nanoseconds and warp-iterations
- * before / after the work queue ran dry, warps, the longest warp, live lanes per iteration */
+/* all 16 counter slots, since the last reset: out[0] = SDF evaluations executed, out[1] = pixel-samples rendered,
+ * out[2] = how many of out[0] took the far-field shortcut of a carved scene (below); [3..11] are filled only by programs
+ * built with RMB_PROFILE=1 in the environment (a measurement aid of the march kernel, see tools/march_timeline.py):
+ * warp-nanoseconds and warp-iterations before / after the work queue ran dry, warps, the longest warp, live lanes per
+ * iteration */
 rmb_status rmb_counters_read_all(rmb_ctx* ctx, uint64_t out[16], int reset);
 /* evaluates the scene's sdf() and material functions at n points: in n*3 floats, out n*17 floats
  * (diffuse rgb, specular rgb, roughness, subsurface, subsurfaceColor rgb, IOR, emission rgb, sdf, 0) */

@@ -23,7 +23,7 @@ EXPORTED_SYMBOLS = [
     "rmb_program_get", "rmb_program_is_live", "rmb_program_source", "rmb_program_kernel_attr", "rmb_uniform_set", "rmb_uniform_set_array",
     "rmb_uniform_matrix4", "rmb_fb_acquire", "rmb_fb_release", "rmb_fb_local_rows", "rmb_fb_global_row",
     "rmb_render_sample", "rmb_present", "rmb_present_device", "rmb_present_async", "rmb_present_wait", "rmb_fb_device_ptr", "rmb_fb_plane_bytes",
-    "rmb_fb_read", "rmb_fb_write", "rmb_fb_copy_to_device", "rmb_counters_read", "rmb_counters_read3", "rmb_counters_read_all", "rmb_program_has_carve", "rmb_probe_carve", "rmb_probe", "rmb_compile_only", "rmb_translate_only", "rmb_host_alloc", "rmb_device_alloc", "rmb_device_free",
+    "rmb_fb_read", "rmb_fb_write", "rmb_fb_copy_to_device", "rmb_counters_read_all", "rmb_program_has_carve", "rmb_probe_carve", "rmb_probe", "rmb_compile_only", "rmb_translate_only", "rmb_host_alloc", "rmb_device_alloc", "rmb_device_free",
     "rmb_host_free", "rmb_measure_fp32_peak", "rmb_measure_fp32x2_peak", "rmb_owned_rows_below",
     "rmb_uniforms_set_frame", "rmb_host_register", "rmb_host_unregister", "rmb_stream_write_u32", "rmb_stream_wait_geq_u32", "rmb_ctx_wait_ctx",
     "rmb_group_create", "rmb_group_destroy", "rmb_group_last_error", "rmb_group_size", "rmb_group_ctx", "rmb_group_sync", "rmb_group_program_get",
@@ -95,8 +95,6 @@ def _load() -> C.CDLL:
         "rmb_fb_read": (i, [vp, vp, i, vp, sz]),
         "rmb_fb_write": (i, [vp, vp, i, vp, sz]),
         "rmb_fb_copy_to_device": (i, [vp, vp, i, vp, sz]),
-        "rmb_counters_read": (i, [vp, C.POINTER(C.c_uint64), i]),
-        "rmb_counters_read3": (i, [vp, C.POINTER(C.c_uint64), i]),
         "rmb_counters_read_all": (i, [vp, C.POINTER(C.c_uint64), i]),
         "rmb_program_has_carve": (i, [vp]),
         "rmb_probe_carve": (i, [vp, vp, vp, i, vp]),

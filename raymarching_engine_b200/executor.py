@@ -160,15 +160,12 @@ class RenderJobContext:                  # RenderJobExecutor.tsx:32-54
         return int(L.rmb_ctx_launch_count(self.handle))
 
     def counters(self, reset: bool = False):
-        out = (C.c_uint64 * 2)()
-        L.rmb_counters_read(self.handle, out, 1 if reset else 0)
-        return int(out[0]), int(out[1])
+        """(SDF evaluations, pixel-samples)"""
+        return tuple(self.counters_all(reset)[:2])
 
     def counters3(self, reset: bool = False):
         """(SDF evaluations, pixel-samples, evaluations that took the far-field shortcut)"""
-        out = (C.c_uint64 * 3)()
-        L.rmb_counters_read3(self.handle, out, 1 if reset else 0)
-        return int(out[0]), int(out[1]), int(out[2])
+        return tuple(self.counters_all(reset)[:3])
 
     def counters_all(self, reset: bool = False):
         """all 16 counter slots (rmb_counters_read_all; slots 3.. are filled by RMB_PROFILE=1 programs only)"""
