@@ -2,7 +2,9 @@
 """One-process sweep of RMB_MARCH_PLAN (rmb_api.cpp "march stage": budget:threads:ctas_per_sm:pause per pass) on the
 default bench workload: frames of the orbit path, one context, L2 flushed per frame, march-kernel time from the
 library's CUDA-event timer and frame time from events around the whole sequence.  The plan is read at every draw, so
-no recompilation is needed between rows.
+no recompilation is needed between rows.  Before a plan is timed, frame 0 of the orbit is rendered under it and its
+RGBA8, depth bits and SDF evaluation count are compared with the first plan's: a plan that differs (lost or repeated
+rays) prints MISMATCH instead of a timing row.
 
   python tools/sweep_plan.py [--width 1920 --height 1080] [--mode preview] [--steps 12] plan [plan ...]
 """
@@ -25,6 +27,7 @@ def main():
     ap.add_argument("--ranks", type=int, default=1, help="emulate one rank of an N-rank row-tile split (rank 0's tiles only): the per-GPU work of --shard tiles")
     ap.add_argument("plans", nargs="+")
     a = ap.parse_args()
+    import numpy as np
     import torch
     import bench
     import raymarching_engine_b200 as rm
@@ -51,9 +54,31 @@ def main():
         assert L.rmb_present_device(ctx.handle, fb.handle, 1.0) == 0
         ctx.fbo.delete(W, H, s.render.frameid)
 
+    def frame0():
+        """RGBA8, depth bits and SDF evaluations of orbit frame 0 under the current plan"""
+        frame[0] += 1
+        s = bench.make_schema(rm, src, custom, W, H, a.mode, 0, frame[0])
+        fb = ctx.fbo.create(W, H, s.render.frameid)
+        rm.upload_sample_uniforms(prog, s, (0.5, 1.0 / 3.0))
+        ctx.counters_all(reset=True)
+        assert L.rmb_render_sample(ctx.handle, prog.handle, fb.handle, 0, 0, W, H) == 0, ctx.last_error()
+        rgba, depth = ctx.present(fb, 1.0)
+        out = (rgba.copy(), depth.view(np.uint32).copy(), ctx.counters_all(reset=True)[0])
+        ctx.fbo.delete(W, H, s.render.frameid)
+        return out
+
     print(f"# {W}x{H} {a.mode} {a.flavour}; ms per frame incl. a 160 MiB L2 flush (~0.05 ms); march = all march launches of a frame")
+    want = None
     for plan in a.plans:
         os.environ["RMB_MARCH_PLAN"] = plan
+        got = frame0()
+        if want is None:
+            want = got
+        elif not (np.array_equal(got[0], want[0]) and np.array_equal(got[1], want[1]) and got[2] == want[2]):
+            px = int(np.any(got[0] != want[0], axis=-1).sum())
+            print(f"{plan:44s} MISMATCH with {a.plans[0]}: {px} RGBA8 pixels and {int((got[1] != want[1]).sum())} depth values "
+                  f"differ, {got[2]} SDF evaluations against {want[2]}", flush=True)
+            continue
         for i in range(4):
             step(i)
         ctx.sync()
