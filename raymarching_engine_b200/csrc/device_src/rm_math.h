@@ -310,6 +310,151 @@ RM_HD float log_f(float x) {
     return (float)(dlog2_pos((double)x) * 6.93147180559945286227e-01);
 }
 
+// ---------------------------------------------------------------- fast paths of the pipeline's RNG functions
+// tan_ft, sincos_ft and log_ft end in a conversion to float: their binary64 value P only has to pick (float)P.
+// For the arguments the RNG produces, each fast path below computes a cheaper binary64 value F - no special-case
+// branches, no correctly rounded division - with |F - P| <= D units in the last place of F, and returns (float)F
+// only when F is farther than D ulps from every float rounding boundary (the midpoint between two floats, where
+// the 29 mantissa bits a float drops read 2^28).  Every value within D ulps of F then rounds to the same float as
+// F, so the result equals the pinned function's by construction.  A binade edge is no rounding boundary, and the
+// nearest boundary across one is 2^24 ulps away, so F and P in neighbouring binades need no special case.  Near a
+// boundary, and outside the domain, the pinned function runs, out of line.  In the tan and log domains every
+// result is a normal float or zero, so F's binade sets the rounding boundaries.  Only IEEE binary64 operations are used (dmul / dadd where an unfused result is meant, whatever
+// --fmad says), so a host build computes the same F: tools/rng_sweep.py checks every float of each domain and
+// measures the largest |F - P|, which D exceeds at least fourfold.
+#if RM_DEVICE_CODE
+#define RM_COLD __device__ __noinline__
+RM_HD double dmul(double a, double b) { return __dmul_rn(a, b); }
+RM_HD double dadd(double a, double b) { return __dadd_rn(a, b); }
+#else
+#define RM_COLD inline
+RM_HD double dmul(double a, double b) { return a * b; }
+RM_HD double dadd(double a, double b) { return a + b; }
+#endif
+struct SinCos { float s, c; };
+RM_COLD float tan_ft_pinned(float x) { return tan_ft(x); }
+RM_COLD SinCos sincos_ft_pinned(float x) { SinCos r; sincos_ft(x, &r.s, &r.c); return r; }
+RM_COLD float log_ft_pinned(float x) { return log_ft(x); }
+
+// F is farther than D ulps (of F) from every float rounding boundary
+RM_HD bool rounds_clear(double F, unsigned D) {
+    const unsigned low = (unsigned)d2ll(F) & 0x1fffffffu;
+    return low - (0x10000000u - D) > 2u * D;
+}
+// n / a for a > 0 normal, within 1 ulp: a bit-pattern estimate of 1/a (relative error < 0.051), three Newton steps
+// (< 2^-34), then one correction of the quotient (error ~ 2^-68 plus its rounding)
+RM_HD double div_pos(double n, double a) {
+    double y = ll2d(0x7FDE623822FC16E6LL - d2ll(a));
+    double e = dfma(-a, y, 1.0);
+    y = dfma(y, e, y);
+    e = dfma(-a, y, 1.0);
+    y = dfma(y, e, y);
+    e = dfma(-a, y, 1.0);
+    y = dfma(y, e, y);
+    const double q = dmul(n, y);
+    return dfma(dfma(-a, q, n), y, q);
+}
+
+// tan_ft on [2^-126, 1024): the pinned reduction (here |x * 2/pi| < 2^31 always takes its first path), then
+// tan r = r + r z P(z) / Q(z), z = r^2, the rational approximation of the Cephes library's tan.c (S. L. Moshier;
+// relative error ~2^-52 on |r| <= pi/4) in place of two polynomials, and the quotient by div_pos.  P and Q are
+// stored negated, so Q > 0.
+#define RM_TAN_FAST_COEFFS                                                                            \
+    1.30936939181383777646e+04, -1.15351664838587416140e+06, 1.79565251976484877988e+07, /* 0 -P */ \
+    -1.36812963470692954678e+04, 1.32089234440210967447e+06, -2.50083801823357915839e+07,            \
+    5.38695755929454629881e+07                                                           /* 3 -Q */
+#if RM_DEVICE_CODE
+__device__ __constant__ double rm_tan_tab[7] = {RM_TAN_FAST_COEFFS};
+#else
+static const double rm_tan_tab[7] = {RM_TAN_FAST_COEFFS};
+#endif
+constexpr unsigned RM_TAN_FAST_D = 16;
+RM_HD double tan_ft_fast_value(float x) {
+    typedef TrigTab K;
+    const double xd = (double)x;
+    const double t = dadd(dmul(xd, K::at(0)), K::at(16));
+    const double k = dadd(t, -K::at(16));
+    double r = dfma(-k, K::at(1), xd);
+    r = dfma(-k, K::at(2), r);
+    r = dfma(-k, K::at(3), r);
+    const double z = dmul(r, r);
+    double p = dfma(z, rm_tan_tab[0], rm_tan_tab[1]);
+    p = dfma(z, p, rm_tan_tab[2]);
+    double q = dadd(-z, rm_tan_tab[3]);
+    q = dfma(z, q, rm_tan_tab[4]);
+    q = dfma(z, q, rm_tan_tab[5]);
+    q = dfma(z, q, rm_tan_tab[6]);
+    const double n = dfma(dmul(r, z), p, dmul(r, q));       // tan r = n / q, n has the sign of r
+    // n / q in even quadrants; -q / n in odd ones, as q / -n so that the divisor is positive
+    const bool odd = (d2ll(t) & 1) != 0;
+    const double num = odd ? (r < 0.0 ? q : -q) : n;
+    const double den = odd ? dabs(n) : q;
+    return div_pos(num, den);
+}
+RM_HD float tan_ft_fast(float x) {
+    if ((unsigned)(f2i(x) - 0x00800000) >= (unsigned)(0x44800000 - 0x00800000)) return tan_ft_pinned(x);
+    const double F = tan_ft_fast_value(x);
+    if (!rounds_clear(F, RM_TAN_FAST_D)) return tan_ft_pinned(x);
+    return (float)F;
+}
+
+// sincos_ft on [+0, 8): the pinned operations without the special cases and the second reduction path, so F == P
+// and no rounding test is needed
+RM_HD void sincos_ft_fast(float x, float* sn, float* cs) {
+    if ((unsigned)f2i(x) >= 0x41000000u) {
+        const SinCos p = sincos_ft_pinned(x);
+        *sn = p.s;
+        *cs = p.c;
+        return;
+    }
+    typedef TrigTab K;
+    const double xd = (double)x;
+    const double t = dadd(dmul(xd, K::at(0)), K::at(16));
+    const double k = dadd(t, -K::at(16));
+    const int q = (int)(d2ll(t) & 3);
+    double r = dfma(-k, K::at(1), xd);
+    r = dfma(-k, K::at(2), r);
+    r = dfma(-k, K::at(3), r);
+    const double ps = ksin<K>(r), pc = kcos<K>(r);
+    double s = (q & 1) ? pc : ps;
+    if (q & 2) s = -s;
+    double c = (q & 1) ? ps : pc;
+    if (((q + 1) & 2) != 0) c = -c;
+    *sn = (float)s;
+    *cs = (float)c;
+}
+
+// log_ft on [2^-126, 1]: the pinned mantissa split, s = f / (2 + f) by div_pos, the atanh series to z^9 (the
+// omitted terms are below 2^-50 of the sum), and ln x = e ln2 + ln m in one fma
+constexpr unsigned RM_LOG_FAST_D = 8;
+RM_HD double log_ft_fast_value(float x) {
+    typedef LeTab K;
+    const long long b = d2ll((double)x);
+    int e = (int)(b >> 52) - 1023;
+    double m = ll2d((b & 0x000fffffffffffffLL) | 0x3ff0000000000000LL);
+    if (m > K::at(13)) { m = dmul(m, 0.5); e += 1; }
+    const double f = dadd(m, -1.0);
+    const double s = div_pos(f, dadd(2.0, f));
+    const double z = dmul(s, s);
+    double p = K::at(3);
+    p = dfma(z, p, K::at(4));
+    p = dfma(z, p, K::at(5));
+    p = dfma(z, p, K::at(6));
+    p = dfma(z, p, K::at(7));
+    p = dfma(z, p, K::at(8));
+    p = dfma(z, p, K::at(9));
+    p = dfma(z, p, K::at(10));
+    p = dfma(z, p, K::at(11));
+    p = dfma(z, p, 1.0);
+    return dfma((double)e, K::at(14), dmul(dadd(s, s), p));
+}
+RM_HD float log_ft_fast(float x) {
+    if ((unsigned)(f2i(x) - 0x00800000) > (unsigned)(0x3f800000 - 0x00800000)) return log_ft_pinned(x);
+    const double F = log_ft_fast_value(x);
+    if (!rounds_clear(F, RM_LOG_FAST_D)) return log_ft_pinned(x);
+    return (float)F;
+}
+
 RM_HD float exp2_f(float x) { return (float)dexp2((double)x); }
 
 RM_HD float exp_f(float x) { return (float)dexp2((double)x * 1.44269504088896338700e+00); }
